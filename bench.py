@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            # the B200 path (C ABI)
   python bench.py --impl reference --steps K --warmup W    # the CPU port of the reference path
+  python bench.py --gpus 1 ... --dump-outputs DIR           # + what the last timed pass computed, DIR/*.npy
 
 One "step" = one full level-0 pass (decode -> Gram -> ridge solves -> out-of-fold predictions
 -> standardised W) over ALL blocks of the workload (BASELINE.json configs[1]: N=100k samples,
@@ -28,6 +29,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the tree may be read-only: nothing is written there
 # Hardware queues for the lane streams of a Step-1 handle: with 32 instead of the driver's default 8 the library runs 12 lanes
 # (csrc/rg_api.cu, rg_step1_create; profiles/ab_r2u_connections_lanes.txt).  The variable is read when the CUDA context is
 # created, i.e. it has to be in the environment before torch touches the device.  A 32-queue context takes ~1 s longer to
@@ -37,6 +39,7 @@ os.environ.setdefault("CUDA_DEVICE_MAX_CONNECTIONS", "32")
 
 SEED = 20260924
 CFG = dict(N=100_000, M=50_000, P=10, C=3, bsize=1000, K=5, R=5, miss=0.01)
+DUMP_BYTES = 48 << 20                    # --dump-outputs: at most this much of W (a fixed, seeded sample of its rows)
 
 
 def load_peaks():
@@ -359,6 +362,8 @@ def run_gpu(args):
     st.sync()
     if st.status() != 0:
         raise SystemExit("level-0 reported an error (timed pass): " + capi.lib().rg_last_error().decode())
+    if args.dump_outputs:
+        dump_level0(st, len(blocks), N, P, R, args.dump_outputs)
     total_snps = M * args.steps * world
     value = total_snps / (ms / 1e3)
 
@@ -558,6 +563,21 @@ def run_gpu(args):
     print(json.dumps(line), flush=True)
     if dist is not None:
         dist.barrier(); dist.destroy_process_group()
+
+
+def dump_level0(st, nblocks, N, P, R, d):
+    """What the last timed pass computed, as a caller of rg_l0_fetch_W receives it: the level-0 predictors W (N x R per
+    block and phenotype).  All of W is nblocks x P x N x R doubles (2 GB for the benchmark), so the same seeded sample of
+    rows is kept from every block: level0_W.npy [nblocks, P, rows, R] float64, the row indices in level0_W_rows.npy."""
+    n_rows = max(1, min(N, DUMP_BYTES // (8 * nblocks * P * R)))
+    rows = np.sort(np.random.default_rng(SEED).choice(N, n_rows, replace=False))
+    W = np.empty((nblocks, P, n_rows, R))
+    for b in range(nblocks):
+        for p in range(P):
+            W[b, p] = st.fetch_W(b, p)[rows]
+    os.makedirs(d, exist_ok=True)
+    np.save(os.path.join(d, "level0_W.npy"), W)
+    np.save(os.path.join(d, "level0_W_rows.npy"), rows.astype(np.float64))
 
 
 def file_e2e_leg(host_panel, N, M, bs, P, Yr, cov, na, gpus=1):
@@ -993,7 +1013,19 @@ def main():
     ap.add_argument("--blocks", type=int, default=0, help="profiling only: restrict the pass to the first n blocks")
     ap.add_argument("--n-samples", type=int, default=0, help="exploration only: other sample count, --blocks blocks (default 20)")
     ap.add_argument("--n-pheno", type=int, default=0, help="exploration only: other trait count (configs[4] has 50)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="after the timed steps, write the level-0 predictors of the last one (a fixed sample of rows) "
+                         "to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and int(os.environ.get("WORLD_SIZE", "1")) > 1:
+        ap.error("--dump-outputs runs on one GPU (sharded, each rank holds the predictors of its own phenotypes only)")
+    from oracle import ref_eigen
+    if args.impl == "b200" and not args.no_cpu and not ref_eigen.available():
+        sys.stderr.write("bench.py: oracle/_ref/libregenie_ref_eigen*.so not built (it needs the reference's sources): "
+                         "running without the CPU baseline and its parity check\n")
+        args.no_cpu = True
     if args.impl == "reference":
         run_reference(args)
     else:

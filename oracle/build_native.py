@@ -29,15 +29,21 @@ PGEN_SHIM = os.path.join(HERE, "ref_pgenlib", "pgen_ref_shim.cpp")
 PGEN_LIB = os.path.join(OUT, "libpgenlib_ref.so")
 
 
+def _skip(name, src):
+    """Without the reference's sources the checker is optional: the tests compare with its stored outputs
+    (tests/golden/ref/) and bench.py leaves out its CPU baseline."""
+    sys.stderr.write("oracle/_ref/%s not built: the reference's sources (%s) are not available\n" % (name, src))
+
+
 def build_pgenlib(verbose=False):
     """The reference's vendored pgenlib, from its own sources where they lie (its Makefile: g++ -O3 -std=c++11 over
     include/*.cc, *.cpp, *.cc with -I simde -I include), plus oracle/ref_pgenlib/pgen_ref_shim.cpp -> oracle/_ref/."""
     import glob
     gxx = shutil.which("g++")
     if not (os.path.isdir(PGENLIB) and gxx):
-        if os.path.exists(PGEN_LIB):
-            return                             # GPU box: the prebuilt checker travels with the snapshot
-        raise RuntimeError("oracle/_ref/libpgenlib_ref.so missing and the reference's pgenlib (%s) is not available" % PGENLIB)
+        if not os.path.exists(PGEN_LIB):
+            _skip("libpgenlib_ref.so", PGENLIB)
+        return                                 # a prebuilt checker is used as it is
     if os.path.exists(PGEN_LIB) and os.path.getmtime(PGEN_LIB) > max(os.path.getmtime(PGEN_SHIM), os.path.getmtime(__file__)):
         return
     os.makedirs(OUT, exist_ok=True)
@@ -60,9 +66,9 @@ def build(verbose=False):
     for name, extra in LIBS.items():
         lib = os.path.join(OUT, name)
         if not have_src:
-            if os.path.exists(lib):
-                continue                       # GPU box: prebuilt checker travels with the snapshot
-            raise RuntimeError("oracle/_ref/%s missing and the reference's Eigen (%s) is not available to build it" % (name, EIGEN))
+            if not os.path.exists(lib):
+                _skip(name, EIGEN)
+            continue                           # a prebuilt checker is used as it is
         if os.path.exists(lib) and os.path.getmtime(lib) > max(os.path.getmtime(SRC), os.path.getmtime(__file__)):
             continue
         os.makedirs(OUT, exist_ok=True)

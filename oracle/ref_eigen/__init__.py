@@ -29,6 +29,10 @@ def _cpu_has(flag):
     return False
 
 
+def available():
+    return any(os.path.exists(os.path.join(_REF, n)) for n in ("libregenie_ref_eigen.so", "libregenie_ref_eigen_avx2.so"))
+
+
 def lib():
     global _lib, _variant
     if _lib is not None:

@@ -752,3 +752,42 @@ def check_no_split_bgen(run, read, tmp_path, golden_dir):
             s = split[k].get(t[2])
             cols = t[12 + 4 * k: 16 + 4 * k]
             assert cols == (["NA"] * 4 if s is None else s[9:13]), (t, s)
+
+
+# ------------------------------------------------------------------- stored outputs of the compiled reference libraries
+REF_GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ref")
+
+
+def ref_golden(name, compute):
+    """What a library of oracle/_ref/ (compiled from the reference's sources by oracle/build_native.py) returned for a
+    test's inputs, stored as tests/golden/ref/<name>.npz: the comparison then needs neither the library nor the reference's
+    sources.  With RG_WRITE_REF_GOLDEN=1 in the environment, `compute()` runs the library and the file is rewritten."""
+    path = os.path.join(REF_GOLDEN, name + ".npz")
+    if os.environ.get("RG_WRITE_REF_GOLDEN") == "1":
+        os.makedirs(REF_GOLDEN, exist_ok=True)
+        np.savez_compressed(path, **compute())
+    with np.load(path) as z:
+        return {k: z[k] for k in z.files}
+
+
+def sha256(a):
+    """Digest of an exact (integer) result, stored in place of arrays too large to keep."""
+    import hashlib
+    return np.frombuffer(hashlib.sha256(np.ascontiguousarray(a).tobytes()).digest(), dtype=np.uint8)
+
+
+def W_digest(W, n_rows=64, seed=0):
+    """Level-0 predictors [P][N x R] too large to store whole: a fixed, seeded set of rows and every column's max |W|."""
+    rows = np.sort(np.random.default_rng(seed).choice(W[0].shape[0], min(W[0].shape[0], n_rows), replace=False))
+    return {"rows": rows, "W": np.stack([w[rows] for w in W]), "absmax": np.stack([np.abs(w).max(axis=0) for w in W])}
+
+
+def W_rel_err(W, ref, prefix=""):
+    """max over phenotypes of |W - W_ref| / max |W_ref| on the stored rows and of the columns' max |W| against the stored
+    ones: both are bounded by the error over the whole matrix."""
+    err = 0.0
+    for p, w in enumerate(W):
+        scale = ref[prefix + "absmax"][p].max()
+        err = max(err, np.abs(w[ref[prefix + "rows"]] - ref[prefix + "W"][p]).max() / scale,
+                  np.abs(np.abs(w).max(axis=0) - ref[prefix + "absmax"][p]).max() / scale)
+    return float(err)

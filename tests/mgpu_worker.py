@@ -13,6 +13,7 @@ import tempfile
 import numpy as np
 import torch
 import torch.distributed as dist
+from torch.distributed.elastic.multiprocessing.errors import record
 
 sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -41,6 +42,7 @@ def run(pb, dev, distributed):
     return out
 
 
+@record                                 # a failing rank's traceback goes into torchrun's error report
 def main():
     rank, world = int(os.environ["RANK"]), int(os.environ["WORLD_SIZE"])
     ngpu = torch.cuda.device_count()

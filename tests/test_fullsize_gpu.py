@@ -3,7 +3,8 @@
 Direct comparison: one full block of each configuration against the compiled Eigen/OpenMP restatement of
 calc_cv_matrices + ridge_level_0 (oracle/ref_eigen: the reference's own SelfAdjointEigenSolver, seconds per block),
 1e-9 relative on every level-0 predictor column - the benchmarked k-fold path at the benchmarked size (16 Cholesky
-panels, 72 Gram tiles, 5 prediction groups, folds of 20 000 / 100 000 samples).
+panels, 72 Gram tiles, 5 prediction groups, folds of 20 000 / 100 000 samples).  The Eigen side is stored
+(tests/golden/ref/, helpers.ref_golden): every column's max |W| and a fixed, seeded sample of 64 rows.
 
 Size-independent identities on top (they hold for the reference's algorithm at any size):
 
@@ -17,6 +18,7 @@ Size-independent identities on top (they hold for the reference's algorithm at a
 import numpy as np
 import pytest
 
+import helpers
 from regenie_b200 import hostprep, synth
 
 pytestmark = pytest.mark.gpu
@@ -39,25 +41,24 @@ def _step1(X, Y, mask, in_an, neff, total_blocks=3):
     return capi.Step1(X, Y, mask, in_an, hostprep.fold_sizes(N, K), lam, neff, N, BS, total_blocks)
 
 
-def _max_rel(W, W_o):
-    return max(float(np.abs(W[p] - W_o[p]).max() / np.abs(W_o[p]).max()) for p in range(len(W_o)))
-
-
 def test_level0_full_block_matches_the_eigen_oracle_at_configs1(panel):
     """The benchmark configuration itself: N = 100k, bsize = 1000, 10 traits, 5 folds x 5 ridge values, 1 % missing
     calls, 2 % missing phenotypes - every one of the 50 predictor columns vs ridge_level_0 (src/Step1_Models.cpp:458-613)."""
-    from oracle import ref_eigen
     g, packed, X, Y, mask, in_an, neff = panel
     h0 = hostprep.ridge_grid(5)
     lam = 50_000 * (1 - h0) / h0
     fsz = hostprep.fold_sizes(N, K)
-    W_o, _ = ref_eigen.l0_block_kfold(packed, N, in_an, X, Y, mask, fsz, lam, neff, int(in_an.sum()))
+
+    def eigen():
+        from oracle import ref_eigen
+        return helpers.W_digest(ref_eigen.l0_block_kfold(packed, N, in_an, X, Y, mask, fsz, lam, neff, int(in_an.sum()))[0])
+    W_o = helpers.ref_golden("level0_eigen_n100k", eigen)
     st = _step1(X, Y, mask, in_an, neff)
     st.l0_block_bed(packed, BS, 1)
     assert st.status() == 0
     W = [st.fetch_W(1, p) for p in range(P)]
     st.close()
-    err = _max_rel(W, W_o)
+    err = helpers.W_rel_err(W, W_o)
     assert err < 1e-9, "level-0 predictors at N=100k, bs=1000 differ from the Eigen oracle: %g" % err
 
 
@@ -110,7 +111,6 @@ def test_level0_block_at_n_500k():
     """BASELINE configs[2] sample count (N = 500 000, bsize = 1000, 10 traits): one block against the Eigen oracle
     (1e-9), plus the size-independent identities - standardisation sums, finite values, bit-identical columns when
     the block is replayed on another lane."""
-    from oracle import ref_eigen
     from regenie_b200 import capi
     n = 500_000
     rng = np.random.default_rng(123)
@@ -121,14 +121,18 @@ def test_level0_block_at_n_500k():
     cov = rng.standard_normal((n, C - 1))
     X, Yr, mask, in_an, neff = hostprep.prepare_qt(Y, cov, None)
     h0 = hostprep.ridge_grid(5)
-    st = capi.Step1(X, Yr, mask, in_an, hostprep.fold_sizes(n, K), 500_000 * (1 - h0) / h0, neff, n, BS, 2)
     packed = synth.pack_bed(g)
+
+    def eigen():
+        from oracle import ref_eigen
+        return helpers.W_digest(ref_eigen.l0_block_kfold(packed, n, in_an, X, Yr, mask, hostprep.fold_sizes(n, K),
+                                                         500_000 * (1 - h0) / h0, neff, int(in_an.sum()))[0])
+    W_o = helpers.ref_golden("level0_eigen_n500k", eigen)
+    st = capi.Step1(X, Yr, mask, in_an, hostprep.fold_sizes(n, K), 500_000 * (1 - h0) / h0, neff, n, BS, 2)
     st.l0_block_bed(packed, BS, 0)
     st.l0_block_bed(packed, BS, 1)
     assert st.status() == 0
-    W_o, _ = ref_eigen.l0_block_kfold(packed, n, in_an, X, Yr, mask, hostprep.fold_sizes(n, K), 500_000 * (1 - h0) / h0,
-                                      neff, int(in_an.sum()))
-    err = _max_rel([st.fetch_W(0, p) for p in range(P)], W_o)
+    err = helpers.W_rel_err([st.fetch_W(0, p) for p in range(P)], W_o)
     assert err < 1e-9, "level-0 predictors at N=500k, bs=1000 differ from the Eigen oracle: %g" % err
     for p in (0, P - 1):
         w = st.fetch_W(0, p)

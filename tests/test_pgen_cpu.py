@@ -65,25 +65,23 @@ def test_pgen_round_trip_all_record_types(tmp_path):
 
 
 # ------------------------------------------------------------------------------------ pinned on the reference's own pgenlib
-def _pgenlib():
-    import pytest
-    from oracle import pgenlib_ref
-    if not pgenlib_ref.available():
-        pytest.skip("oracle/_ref/libpgenlib_ref.so not built (needs /root/reference/external_libs/pgenlib)")
-    return pgenlib_ref
-
-
+# What pgenlib returned is stored as digests (tests/golden/ref/, helpers.ref_golden): the bytes of each file it validated
+# and of the calls it read from it.
 def test_oracle_equals_pgenlib_on_the_reference_fixture(golden_dir):
     """oracle/pgen.py vs the reference's vendored pgenlib, called as the reference calls it (ReadHardcalls, allele 1)."""
-    ref = _pgenlib()
     path = golden_dir + "/example.pgen"
-    ref.validate(path)
-    want = ref.read_hardcalls(path, 500, 0, 1000)
+
+    def pgenlib():
+        from oracle import pgenlib_ref as ref
+        ref.validate(path)
+        return {"pgen": helpers.sha256(np.fromfile(path, dtype=np.uint8)),
+                "calls": helpers.sha256(ref.read_hardcalls(path, 500, 0, 1000))}
+    want = helpers.ref_golden("pgenlib_example", pgenlib)
+    assert np.array_equal(helpers.sha256(np.fromfile(path, dtype=np.uint8)), want["pgen"])
     pg = pgen.Pgen(path)
-    for v in range(1000):
-        g = pg.read(v).astype(float)
-        g[g == 3] = -3.0
-        assert np.array_equal(g, want[v]), v
+    got = np.stack([pg.read(v).astype(float) for v in range(1000)])
+    got[got == 3] = -3.0
+    assert np.array_equal(helpers.sha256(got), want["calls"])
 
 
 def test_synthetic_files_pass_pgenlib_validation_and_read_back(tmp_path):
@@ -91,19 +89,33 @@ def test_synthetic_files_pass_pgenlib_validation_and_read_back(tmp_path):
     (record types, difflist group byte counts, trailing bits) and ReadHardcalls returns the calls that were written - with
     all samples and with a sample subset (pgenlib's proper-subset readers skip difflist groups by their byte counts) - and
     oracle/pgen.py agrees.  Covers difflists of > 32 groups and 1 / 2 / 3-byte sample ids, which the fixture does not."""
-    ref = _pgenlib()
     from test_host_cpu import big_pgen_calls
-    for N, M, storage in ((700, 160, 5), (33333, 40, 6), (70001, 20, 2)):
+    cases = ((700, 160, 5), (33333, 40, 6), (70001, 20, 2))
+    files = {}
+    for N, M, storage in cases:
         g = synthetic_calls() if N == 700 else big_pgen_calls(N, M)
         pfx = str(tmp_path / ("s%d" % N))
         types = helpers.write_pgen(pfx, g, storage=storage)
         assert set(types) >= set(range(8))
-        ref.validate(pfx + ".pgen")
+        sub = np.sort(np.random.default_rng(N).choice(g.shape[1], g.shape[1] // 3, replace=False))
+        files[N] = (g, pfx + ".pgen", sub)
+
+    def pgenlib():
+        from oracle import pgenlib_ref as ref
+        out = {}
+        for N, (g, path, sub) in files.items():
+            ref.validate(path)
+            out["pgen%d" % N] = helpers.sha256(np.fromfile(path, dtype=np.uint8))
+            out["calls%d" % N] = helpers.sha256(ref.read_hardcalls(path, g.shape[1], 0, g.shape[0]))
+            out["subset%d" % N] = helpers.sha256(ref.read_hardcalls(path, g.shape[1], 0, g.shape[0], subset=sub))
+        return out
+    ref = helpers.ref_golden("pgenlib_synthetic", pgenlib)
+    for N, (g, path, sub) in files.items():
+        assert np.array_equal(helpers.sha256(np.fromfile(path, dtype=np.uint8)), ref["pgen%d" % N]), N
         want = g.astype(float)
         want[want == 3] = -3.0
-        assert np.array_equal(ref.read_hardcalls(pfx + ".pgen", g.shape[1], 0, g.shape[0]), want)
-        sub = np.sort(np.random.default_rng(N).choice(g.shape[1], g.shape[1] // 3, replace=False))
-        assert np.array_equal(ref.read_hardcalls(pfx + ".pgen", g.shape[1], 0, g.shape[0], subset=sub), want[:, sub])
-        pg = pgen.Pgen(pfx + ".pgen")
+        assert np.array_equal(helpers.sha256(want), ref["calls%d" % N]), N
+        assert np.array_equal(helpers.sha256(want[:, sub]), ref["subset%d" % N]), N
+        pg = pgen.Pgen(path)
         for v in (list(range(g.shape[0])) + [g.shape[0] - 1, 3, 1]):
             assert np.array_equal(pg.read(v), g[v]), (N, v)
